@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- the headline measurement (BASELINE.json metric) of the B200-native LightCTR hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload fm_c2|ffm_c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload fm_c2|ffm_c3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (gather -> interaction -> loss -> scatter-add -> updater) over one batch of
 synthetic Criteo-shaped input.  N=1 workload = BASELINE.json configs[1]: FM k=16, 1M features, 39 fields,
 ~77 nnz/row, batch 4096, Adagrad.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (float32; see dump_outputs), so that two
+builds run with the same arguments -- hence the same seeded inputs -- can be compared output for output.
+The benchmark reads the library build() compiled and writes nothing into the tree.
 """
 import argparse
 import ctypes as C
@@ -220,7 +224,34 @@ def check_against_oracle(ctx, wl, batch, Fc):
     return out
 
 
-def measure(wname, wl, args, rank, world, local_rank, dist, steps, warmup, do_e2e=True, split_global=0):
+DUMP_MAX_BYTES = 64 << 20
+DUMP_RANDOM_ROWS = 65536
+
+
+def dump_outputs(ctx, wl, batch, slot, out_dir):
+    """Write what the last timed step handed its caller: the batch's pCTR (`pred`), and the parameter rows W[rows] (`W_rows`)
+    and V[rows] (`V_rows`, one row of the factor table per id) after the update.  `rows` is the sorted union of the ids the
+    step read and updated and a fixed seeded sample of all ids (mostly ids the step must leave unchanged), trimmed by the
+    same seeded draw to keep the files under DUMP_MAX_BYTES; NFM adds its dense layers (`mlp<l>_weight`, `mlp<l>_bias`)."""
+    W, V = ctx.download_params()
+    F, rowlen = wl["F"], ctx.rowlen
+    rng = np.random.default_rng(0)
+    rows = np.union1d(batch[1].astype(np.int64), rng.choice(F, min(F, DUMP_RANDOM_ROWS), replace=False))
+    cap = (DUMP_MAX_BYTES // 2) // (4 * (rowlen + 1))
+    if len(rows) > cap:
+        rows = np.sort(rng.choice(rows, cap, replace=False))
+    out = {"pred": ctx.download_pred(slot), "W_rows": W[rows], "V_rows": V.reshape(F, rowlen)[rows]}
+    if wl["model"] == "nfm":
+        dims = [wl["k"]] + list(wl["hidden"]) + [1]
+        for li in range(len(dims) - 1):
+            out["mlp%d_weight" % li], out["mlp%d_bias" % li] = ctx.mlp_download(li, dims[li], dims[li + 1])
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
+def measure(wname, wl, args, rank, world, local_rank, dist, steps, warmup, do_e2e=True, split_global=0, dump_dir=None):
     """One workload on this process group: K device-timed steps on resident batches (+ the end-to-end arm)."""
     import torch
     from lightctr_b200 import capi
@@ -307,6 +338,8 @@ def measure(wname, wl, args, rank, world, local_rank, dist, steps, warmup, do_e2
         dist.barrier()
     t_wall = time.time() - t_wall0
     launches = ctx.launch_count() - launches0
+    if dump_dir:
+        dump_outputs(ctx, wl_b, batches[(steps - 1) % NB], (steps - 1) % NB, dump_dir)
     ctx.profile(True)
     ctx.profile_read(reset=True)
     for i in range(steps):
@@ -397,7 +430,11 @@ def main():
     ap.add_argument("--check", action="store_true", help="compare step 0 of the benched batch with the CPU oracle")
     ap.add_argument("--batch", type=int, default=0, help="override the workload's rows per GPU per step (sweeps; "
                     "the headline configs are the defaults)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -427,8 +464,8 @@ def main():
         return 0
 
     import torch
-    from lightctr_b200 import build as lbuild
-    lbuild.build()
+    from lightctr_b200 import capi
+    capi.load_library()  # the library build() compiled; raises when it is missing
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the product has no CPU path)")
     torch.cuda.set_device(local_rank)
@@ -436,7 +473,7 @@ def main():
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    m = measure(wname, wl, args, rank, world, local_rank, dist, args.steps, args.warmup)
+    m = measure(wname, wl, args, rank, world, local_rank, dist, args.steps, args.warmup, dump_dir=args.dump_outputs)
     value, ms_per_step, prof, B, Fc, det, nnz_mean = m["value"], m["ms_per_step"], m["prof"], m["B"], m["Fc"], m["det"], m["nnz_mean"]
     mlp_bf16 = m["mlp_bf16"]
     k = wl["k"]

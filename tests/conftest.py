@@ -7,8 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REF_DATA = "/root/reference/data"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
@@ -19,10 +17,3 @@ def oracle_api():
     from oracle import api
     api.build(ref=True)
     return api
-
-
-def has_reference():
-    return os.path.isdir(REF_DATA)
-
-
-needs_reference = pytest.mark.skipif(not has_reference(), reason="/root/reference not present (GPU box)")
